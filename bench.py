@@ -2,7 +2,7 @@
 """bench.py -- train tree-clouds/sec of the PointNet++ biomass regressor hot path on B200.
 
     python bench.py --gpus N --steps K --warmup W [--precision bf16|fp32] [--impl reference]
-                    [--config train|eval|dense]
+                    [--config train|eval|dense] [--dump-outputs DIR]
 
 A "step" is one pass of /root/reference/main.py:150-172 over one batch of synthetic tree clouds
 (forward + weighted MSE + backward + gradient all-reduce + Adam), BASELINE.json configs[1]:
@@ -23,11 +23,14 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+# the benchmark writes nothing into the tree it runs from (which may be read-only), bytecode caches included
+sys.dont_write_bytecode = True
 
 import torch  # noqa: E402
 
 METRIC = "train tree-clouds/sec @10k pts"
 UNIT = "tree-clouds/s"
+DUMP_LIMIT_BYTES = 64 * 2 ** 20
 
 
 def parse_args():
@@ -60,6 +63,8 @@ def parse_args():
                     help="N>1: all-reduce the buckets after backward on the training stream instead of on a side stream as "
                          "backward finishes them (measured at N=2: 2.38 ms/step overlapped, 2.41 serial)")
     ap.add_argument("--no-fp32", action="store_true", help="skip the fp32-mode sibling measurement (N=1, train config)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
     if args.config == "dense":
         if args.batch == 12:
@@ -146,12 +151,30 @@ def batch_h2d_bytes(b, with_batch_vector=True):
     return sum(t.numel() * t.element_size() for t in ts if t is not None)
 
 
+def dump_outputs(out_dir, arrays):
+    """Write every tensor of `arrays` as out_dir/<name>.npy, float64 as float64 and everything else as float32.  The
+    inputs depend on the arguments only, so two builds run with the same arguments can be compared file by file.
+
+    A training step hands its caller the loss, so the training configs write that and not the parameters: those differ
+    between two runs of the same build by far more than the loss does (DESIGN.md section 6)."""
+    import numpy as np
+    host = {}
+    for name, t in arrays.items():
+        t = t.detach().cpu()
+        host[name] = (t if t.dtype == torch.float64 else t.float()).numpy()
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------
 #  CPU arm: the reference's CPU path as restated by oracle/ (torch CPU + C fps/radius)
 # ------------------------------------------------------------------------------------------------
-def cpu_train_steps(args, steps, warmup, max_step_s=12.0):
-    """`steps` timed training steps of the oracle network on ALL host cores, every step on the FULL configured batch
-    (the sample is bounded through the number of steps, never through the batch)."""
+def cpu_train_steps(args, steps, warmup):
+    """`steps` timed training steps of the oracle network on ALL host cores, every step on the FULL configured batch."""
     from oracle import ref
     torch.set_num_threads(os.cpu_count() or 1)
     from dl_biomass_b200.data import Batch, synthetic_clouds
@@ -160,6 +183,7 @@ def cpu_train_steps(args, steps, warmup, max_step_s=12.0):
     if args.config == "dense":
         net.sa1_module.r, net.sa2_module.r = 4.0, 16.0
     opt = ref.make_adam(net.parameters())
+    last = {}
 
     def one(i):
         b = Batch.from_data_list(synthetic_clouds(1234 + i * args.batch, args.batch, args.points, 1, False))
@@ -168,18 +192,16 @@ def cpu_train_steps(args, steps, warmup, max_step_s=12.0):
         loss = ref.weighted_mse(net(b), b.y)
         loss.backward()
         opt.step()
+        last["loss"] = loss
         return time.perf_counter() - t0
 
-    t_first = one(0)  # also serves as the first warm-up step
-    for i in range(1, warmup):
+    for i in range(max(warmup, 1)):
         one(i)
-    if t_first > max_step_s:  # a very slow box: fewer steps, never fewer clouds per step
-        steps = max(1, min(steps, int(150.0 / t_first)))
     ts = [one(100 + i) for i in range(steps)]
     total = sum(ts)
     return {"value": args.batch * steps / total, "ms_per_step": 1e3 * total / steps, "steps": steps,
             "clouds_per_step": args.batch, "cores": torch.get_num_threads(), "host_cores": os.cpu_count(),
-            "oracle_threads": ref.num_threads()}
+            "oracle_threads": ref.num_threads(), "loss": last["loss"]}
 
 
 def workload_name(args, precision=None):
@@ -215,6 +237,8 @@ def run_reference(args):
     if rank != 0:
         return
     r = cpu_train_steps(args, args.steps, args.warmup)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"loss": r["loss"].reshape(1)})
     sample = (f"{r['steps']} timed steps (after {args.warmup} warm-up), each a full train step (fwd+loss+bwd+Adam) on "
               f"{r['clouds_per_step']} clouds x {args.points} pts")
     line = {"impl": "reference", "metric": metric_name(args) if args.config != "eval" else METRIC,
@@ -312,14 +336,15 @@ def run_b200(args):
         torch.cuda.synchronize(dev)
 
     def timed(step_fn, steps):
-        """Per-step CUDA events on the current stream, L2 flushed (untimed) before every step."""
-        evs = []
+        """Per-step CUDA events on the current stream, L2 flushed (untimed) before every step.  Returns the summed time
+        and what the last step returned."""
+        evs, last = [], None
         barrier()
         for i in range(steps):
             flush.zero_()
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record()
-            step_fn(i)
+            last = step_fn(i)
             b.record()
             evs.append((a, b))
         barrier()
@@ -327,7 +352,7 @@ def run_b200(args):
         t = torch.tensor([ms], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return float(t.item())
+        return float(t.item()), last
 
     use_graph = not args.no_graph and not (world > 1 and args.dp_mode == "eager")
     # dense clouds (100k points): farthest-point sampling runs one 16-CTA cluster per cloud -- 128 of the 148 SMs for
@@ -360,16 +385,18 @@ def run_b200(args):
             return graphed(batch) if graphed is not None else train_step(net, opt, batch, reducer)
         return net, opt, reducer, stepper, graphed, run_step
 
-    def measure_training(run_step, stepper, graphed, steps, warmup, sample_clocks):
+    def measure_training(run_step, stepper, graphed, steps, warmup, sample_clocks, dump=None):
         def step_resident(i):
-            run_step(pool_dev[(i + 1) % len(pool_dev)])
+            return run_step(pool_dev[(i + 1) % len(pool_dev)])
         for i in range(warmup):
             step_resident(i)
         sampler = ClockSampler(local_rank) if (sample_clocks and rank == 0) else None
         l0 = lib.b2pn_launch_count()
-        total_ms = timed(step_resident, steps)
+        total_ms, last_loss = timed(step_resident, steps)
         launches = lib.b2pn_launch_count() - l0
         clocks = sampler.stop() if sampler else None
+        if dump is not None:   # before the e2e steps below train the model further
+            dump(last_loss)
         if stepper is not None and use_graph:  # replayed kernels do not pass through the library's launch counter
             launches = stepper.launches_per_step * steps
         elif graphed is not None:
@@ -385,7 +412,7 @@ def run_b200(args):
             loss_host.copy_(loss, non_blocking=True)
         for i in range(3):
             step_e2e(i)
-        e2e_ms = timed(step_e2e, steps)
+        e2e_ms, _ = timed(step_e2e, steps)
         return total_ms, e2e_ms, int(launches), clocks
 
     hbm_peak, tc_peak, peak_kind = measured_peaks()
@@ -412,13 +439,15 @@ def run_b200(args):
         torch.cuda.reset_peak_memory_stats(dev)
         sampler = ClockSampler(local_rank) if rank == 0 else None
         l0 = lib.b2pn_launch_count()
-        total_ms = timed(fwd, args.steps)
+        total_ms, out = timed(fwd, args.steps)
         launches = int(lib.b2pn_launch_count() - l0)
         clocks = sampler.stop() if sampler else None
         peak_gb = torch.cuda.max_memory_allocated(dev) / 2 ** 30
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {"out": out})
         for i in range(2):
             fwd_e2e(i)
-        e2e_ms = timed(fwd_e2e, args.steps)
+        e2e_ms, _ = timed(fwd_e2e, args.steps)
         if rank == 0:
             value = world * args.batch * args.steps / (total_ms * 1e-3)
             line = {"metric": metric_name(args), "value": round(value, 2), "unit": UNIT, "n_gpus": world, "steps": args.steps,
@@ -439,7 +468,11 @@ def run_b200(args):
 
     # =============================================================================================================
     net, opt, reducer, stepper, graphed, run_step = build_training(precision)
-    total_ms, e2e_ms, launches, clocks = measure_training(run_step, stepper, graphed, args.steps, warmup, True)
+
+    def dump(loss):
+        dump_outputs(args.dump_outputs, {"loss": loss.reshape(1)})
+    total_ms, e2e_ms, launches, clocks = measure_training(run_step, stepper, graphed, args.steps, warmup, True,
+                                                          dump if args.dump_outputs and rank == 0 else None)
     value = world * args.batch * args.steps / (total_ms * 1e-3)
     e2e_value = world * args.batch * args.steps / (e2e_ms * 1e-3)
     sm_limit_note = stepper.sm_limit if stepper is not None else 0
@@ -518,7 +551,7 @@ def run_b200(args):
         del net, opt, stepper, graphed, run_step
         torch.cuda.empty_cache()
         netf, optf, _, stepf, graphf, runf = build_training("fp32")
-        k = max(3, min(args.steps, 10))
+        k = args.steps
         t_ms, e_ms, lf, _ = measure_training(runf, stepf, graphf, k, 3, False)
         if stepf is not None:
             stepf.close()

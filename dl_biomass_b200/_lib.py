@@ -8,6 +8,7 @@ from __future__ import annotations
 
 import ctypes
 import os
+import shutil
 import subprocess
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -98,9 +99,15 @@ SIGNATURES = {
 }
 
 
+def cuda_tool(name: str) -> str:
+    """Path of a CUDA toolkit program: from PATH, else from $CUDA_HOME/bin (default /usr/local/cuda), since an ordinary
+    user's PATH need not hold the toolkit."""
+    return shutil.which(name) or os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", name)
+
+
 def build(force: bool = False, verbose: bool = False) -> str:
     """Compile libb2pn.so in-tree with nvcc for sm_100a (works without a GPU)."""
-    cmd = ["make", "-C", CSRC, "-j8"] + (["-B"] if force else [])
+    cmd = ["make", "-C", CSRC, "-j8", f"NVCC={cuda_tool('nvcc')}"] + (["-B"] if force else [])
     res = subprocess.run(cmd, capture_output=True, text=True)
     if verbose or res.returncode != 0:
         print(res.stdout[-4000:], res.stderr[-4000:])

@@ -81,7 +81,10 @@ def gen_grouping_oracle():
         idx2 = ref.fps_ref(pos1, ptr1, 0.25)
         ptr2 = ref.sample_ptr(ptr1, 0.25)
         nbr2, cnt2 = ref.ball_query_ref(pos1, pos1[idx2], ptr1, ptr2, r2, 64)
-        out.update({f"spec_{i}": np.array([seed, B, n, int(ragged), r1, r2]), f"idx1_{i}": idx1.numpy(),
+        # the clouds themselves are stored: torch's CPU normal sampler gives different bits on different CPUs (vector
+        # vs scalar kernels), so re-drawing them from the seed would make the fixture depend on the host
+        out.update({f"spec_{i}": np.array([seed, B, n, int(ragged), r1, r2]), f"pos_{i}": b.pos.numpy(),
+                    f"ptr_{i}": b.ptr.numpy(), f"idx1_{i}": idx1.numpy(),
                     f"cnt1_{i}": cnt1.numpy(), f"nbr1_{i}": nbr1.numpy(), f"idx2_{i}": idx2.numpy(),
                     f"cnt2_{i}": cnt2.numpy(), f"nbr2_{i}": nbr2.numpy()})
     np.savez_compressed(os.path.join(GOLD, "grouping_oracle.npz"), **out)
@@ -89,11 +92,16 @@ def gen_grouping_oracle():
 
 
 def gen_net_oracle():
+    # the input clouds are stored (see gen_grouping_oracle), and the network runs in float64: in float32 its train-mode
+    # gradients of levels 1-2 (BatchNorm backward over few rows) move by up to ~0.5 % with the host's summation order
+    # (thread count, CPU kernels), which a fixture must not pin
     torch.manual_seed(0)
-    b = Batch.from_data_list(synthetic_clouds(4321, 3, 768, 1, True))
+    clouds = synthetic_clouds(4321, 3, 768, 1, True)
+    b = Batch.from_data_list(clouds)
+    b.x, b.pos = b.x.double(), b.pos.double()
     res = {}
     for mode in ("train", "eval"):
-        net = ref.seeded_init_(ref.NetRef(1, "ReLU", 0, 0.0), seed=7)
+        net = ref.seeded_init_(ref.NetRef(1, "ReLU", 0, 0.0), seed=7).double()
         net.train(mode == "train")
         out = net(b)
         loss = ref.weighted_mse(out, b.y)
@@ -111,7 +119,8 @@ def gen_net_oracle():
                        "grad_digest": {k: digest(v) for k, v in r["grads"].items()},
                        "grad_head": {k: v.flatten()[:16].clone() for k, v in r["grads"].items()},
                        "buf_digest": {k: digest(v.float()) for k, v in r["buffers"].items()}}
-    torch.save({"spec": (4321, 3, 768, 1, True), "init_seed": 7, "modes": small}, os.path.join(GOLD, "net_oracle.pt"))
+    torch.save({"spec": (4321, 3, 768, 1, True), "init_seed": 7, "modes": small,
+                "clouds": [{"x": c.x, "pos": c.pos, "y": c.y} for c in clouds]}, os.path.join(GOLD, "net_oracle.pt"))
     print("net_oracle.pt: out(train) =", res["train"]["out"].flatten()[:4])
 
 

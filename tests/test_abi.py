@@ -80,7 +80,8 @@ def test_cpu_tensors_fail_loudly(built_lib):
 
 def test_grouping_sass_has_no_fma(built_lib):
     """Distances must be ((dx*dx+dy*dy)+dz*dz) with separate roundings (SURVEY.md A.7)."""
-    sass = subprocess.run(["cuobjdump", "-sass", built_lib.LIB_PATH], capture_output=True, text=True).stdout
+    sass = subprocess.run([built_lib.cuda_tool("cuobjdump"), "-sass", built_lib.LIB_PATH], capture_output=True,
+                          text=True).stdout
     cur, bad = None, []
     for line in sass.splitlines():
         m = re.search(r"Function : (\S+)", line)

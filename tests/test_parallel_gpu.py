@@ -130,7 +130,7 @@ def _local_grads(rank, dev):
 @pytest.mark.parametrize("mode", ["split", "captured"])
 def test_world2_nccl_replicas_stay_identical(cuda_device, tmp_path, mode):
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (run under gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     ctx = mp.start_processes(_rank_worker, args=(2, _free_port(), str(tmp_path), mode), nprocs=2, join=False,
                              start_method="spawn")
     import time

@@ -7,7 +7,7 @@ import torch
 
 from oracle import ref
 from dl_biomass_b200 import ops, sa
-from dl_biomass_b200.data import Batch, synthetic_clouds
+from dl_biomass_b200.data import Batch, Data, synthetic_clouds
 from dl_biomass_b200.pointnet2_regressor import MLP, Net
 
 pytestmark = pytest.mark.gpu
@@ -129,8 +129,7 @@ def test_net_forward_backward_fp32_vs_oracle(cuda_device, train):
 
 def test_net_matches_golden_fixture(cuda_device):
     gold = torch.load(os.path.join(GOLD, "net_oracle.pt"))
-    seed, B, n, F, ragged = gold["spec"]
-    b = Batch.from_data_list(synthetic_clouds(seed, B, n, F, ragged))
+    b = Batch.from_data_list([Data(**c) for c in gold["clouds"]])   # the stored clouds
     for mode in ("train", "eval"):
         _, net = _net_pair(cuda_device, "fp32", mode == "train")
         out = net(b.to(cuda_device))
