@@ -212,8 +212,14 @@ typedef struct b2pn_sa_args {
     int32_t deterministic;       /* PREC_BF16 backward.  0: the row splits of a dW GEMM add their partial sums into one
                                     buffer with fp32 atomics (red.global.add.v4.f32): fastest, last bits vary from run to
                                     run (as in the reference's scatter / cuBLAS kernels).  1: per-split partials summed
-                                    in a fixed order and the grad_x scatter done by one owner per source row: bit-
-                                    reproducible gradients                                                            */
+                                    in a fixed order and the grad_x scatter of SLOTS levels accumulated in 64-bit fixed
+                                    point: bit-reproducible gradients.
+                                    Range of that accumulator: unit 2^-40, every fp32 addend rounded to it (absolute
+                                    error <= 2^-41 ~ 4.5e-13 per addend; addends below that vanish) and every partial
+                                    sum of one grad_x element held in |sum| < 2^23 ~ 8.4e6.  For the result to stay
+                                    within 16-bit accuracy (~4e-3 relative) the typical addend must exceed ~1e-10;
+                                    the level-2 addends of a bf16 training step (3 x 640 points) span 8e-10 .. 8e-2,
+                                    median 1.6e-3; tests/test_sa_pinned_gpu.py sweeps grad_out over 2^-24 .. 2^12   */
     void *out_bf16;              /* PREC_BF16, optional: a 16-bit (fp16) copy of `out` [n_dst, c3] written by the same epilogue --
                                     the next level's gather reads it (half the bytes, no separate cast kernel)         */
 } b2pn_sa_args;

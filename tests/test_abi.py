@@ -64,7 +64,7 @@ def test_product_never_imports_oracle():
 def test_oracle_never_imports_product():
     """The oracle is an independent restatement: oracle/ref.py and oracle/augment_ref.py must not lean on the package they
     check (the golden-vector generator scripts may use its synthetic-cloud helper)."""
-    for f in ("ref.py", "augment_ref.py", "b2pn_oracle.c"):
+    for f in ("ref.py", "augment_ref.py", "sa_pinned.py", "b2pn_oracle.c"):
         txt = open(os.path.join(ROOT, "oracle", f)).read()
         assert not re.search(r"^\s*(from|import)\s+dl_biomass_b200\b", txt, flags=re.M), f
         assert "libb2pn.so" not in txt, f
