@@ -16,7 +16,7 @@ LIB_PATH = os.path.join(_HERE, "libb2pn.so")
 CSRC = os.path.join(_HERE, "csrc")
 
 _lib = None
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 _vp, _i32, _i64, _f32, _f64 = ctypes.c_void_p, ctypes.c_int32, ctypes.c_int64, ctypes.c_float, ctypes.c_double
 
@@ -85,7 +85,6 @@ SIGNATURES = {
     "b2pn_sa_workspace_bytes": (_i64, [ctypes.POINTER(SaArgs), _i32]),
     "b2pn_sa_forward": (ctypes.c_int, [ctypes.POINTER(SaArgs), _vp]),
     "b2pn_sa_eval_fused": (ctypes.c_int, [ctypes.POINTER(SaArgs)]),
-    "b2pn_sa_train_chained": (ctypes.c_int, [ctypes.POINTER(SaArgs)]),
     "b2pn_augment_batch": (ctypes.c_int, [_vp, _vp, ctypes.c_int32, ctypes.POINTER(AugmentCloud), ctypes.c_int32,
                                           ctypes.c_uint64, _vp, _vp, _vp, _vp, _vp]),
     "b2pn_augment_draw": (ctypes.c_uint64, [ctypes.c_uint64, ctypes.c_uint64, ctypes.c_uint32, ctypes.c_uint64]),

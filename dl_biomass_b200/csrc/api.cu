@@ -5,26 +5,7 @@
 
 namespace b2pn {
 long long g_launches = 0;
-thread_local int t_sm_limit = 0;
-thread_local int t_deterministic = 0;
 }
-
-namespace {
-// copies the per-call options of one b2pn_sa_* call into the calling thread's slots for its duration
-struct CallOptions {
-    int prev_limit, prev_det;
-    explicit CallOptions(const b2pn_sa_args &a) : prev_limit(b2pn::t_sm_limit), prev_det(b2pn::t_deterministic)
-    {
-        b2pn::t_sm_limit = a.sm_limit > 0 ? a.sm_limit : 0;
-        b2pn::t_deterministic = a.deterministic ? 1 : 0;
-    }
-    ~CallOptions()
-    {
-        b2pn::t_sm_limit = prev_limit;
-        b2pn::t_deterministic = prev_det;
-    }
-};
-}  // namespace
 
 extern "C" int b2pn_abi_version(void) { return B2PN_ABI_VERSION; }
 
@@ -58,7 +39,6 @@ int64_t sa_workspace_bytes_bf16(const b2pn_sa_args &a, int backward);
 int sa_forward_bf16(const b2pn_sa_args &a, cudaStream_t st);
 int sa_gather_rows_bf16(const b2pn_sa_args &a, cudaStream_t st);
 int sa_eval_fused_bf16(const b2pn_sa_args &a);
-int sa_train_chained_bf16(const b2pn_sa_args &a);
 int sa_backward_bf16(const b2pn_sa_args &a, const b2pn_sa_grads &g, cudaStream_t st);
 }  // namespace tc
 }  // namespace b2pn
@@ -67,7 +47,6 @@ extern "C" int64_t b2pn_sa_workspace_bytes(const b2pn_sa_args *args, int32_t bac
 {
     if (!args) return B2PN_EINVAL;
     if (args->sm_limit < 0) return B2PN_EINVAL;
-    const CallOptions opts(*args);
     if (args->precision == B2PN_PREC_F32) return b2pn::simt::sa_workspace_bytes_f32(*args, backward);
     if (args->precision == B2PN_PREC_BF16) return b2pn::tc::sa_workspace_bytes_bf16(*args, backward);
     return B2PN_ENOTSUP;
@@ -77,7 +56,6 @@ extern "C" int b2pn_sa_forward(const b2pn_sa_args *args, b2pn_stream_t stream)
 {
     if (!args) return B2PN_EINVAL;
     if (args->sm_limit < 0) return B2PN_EINVAL;
-    const CallOptions opts(*args);
     if (args->precision == B2PN_PREC_F32) return b2pn::simt::sa_forward_f32(*args, (cudaStream_t)stream);
     if (args->precision == B2PN_PREC_BF16) return b2pn::tc::sa_forward_bf16(*args, (cudaStream_t)stream);
     return B2PN_ENOTSUP;
@@ -90,17 +68,9 @@ extern "C" int b2pn_sa_eval_fused(const b2pn_sa_args *args)
     return b2pn::tc::sa_eval_fused_bf16(*args);
 }
 
-extern "C" int b2pn_sa_train_chained(const b2pn_sa_args *args)
-{
-    if (!args) return B2PN_EINVAL;
-    if (args->precision != B2PN_PREC_BF16) return 0;
-    return b2pn::tc::sa_train_chained_bf16(*args);
-}
-
 extern "C" int b2pn_sa_gather_rows(const b2pn_sa_args *args, b2pn_stream_t stream)
 {
     if (!args) return B2PN_EINVAL;
-    const CallOptions opts(*args);
     if (args->precision == B2PN_PREC_BF16) return b2pn::tc::sa_gather_rows_bf16(*args, (cudaStream_t)stream);
     return B2PN_ENOTSUP;  // the fp32 kernels gather inside their loaders
 }
@@ -109,7 +79,6 @@ extern "C" int b2pn_sa_backward(const b2pn_sa_args *args, const b2pn_sa_grads *g
 {
     if (!args || !grads) return B2PN_EINVAL;
     if (args->sm_limit < 0) return B2PN_EINVAL;
-    const CallOptions opts(*args);
     if (args->precision == B2PN_PREC_F32) return b2pn::simt::sa_backward_f32(*args, *grads, (cudaStream_t)stream);
     if (args->precision == B2PN_PREC_BF16) return b2pn::tc::sa_backward_bf16(*args, *grads, (cudaStream_t)stream);
     return B2PN_ENOTSUP;

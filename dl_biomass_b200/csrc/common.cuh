@@ -27,11 +27,6 @@ typedef unsigned long long u64;
 
 // number of kernels this library has enqueued (bench.py reports it as gpu_launches)
 extern long long g_launches;
-// per-CALL launch options of the set-abstraction entry points (b2pn_sa_args::sm_limit / ::deterministic): the entry
-// point copies them into these thread-local slots for the helpers below it, so two host threads driving two GPUs (the
-// reference's thread-per-GPU DataParallel, /root/reference/main.py:140) never see each other's settings
-extern thread_local int t_sm_limit;       // upper bound on the CTAs of the persistent tcgen05 kernels (0 = every SM)
-extern thread_local int t_deterministic;  // 1: fixed-order reduction of the dW split partials (bit-reproducible)
 // cudaFuncAttributeMaxDynamicSharedMemorySize is a per-(kernel, device) property: raise it once, not on every launch
 // (invisible under CUDA graphs, but ~1 us of host time per launch in the eager, ragged-batch training loop).
 // `slot`: one static per call site (per kernel instantiation): the largest size set so far per device.

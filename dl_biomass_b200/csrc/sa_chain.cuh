@@ -389,7 +389,7 @@ __global__ void __launch_bounds__(CH_THREADS, 1) tc_chain_eval_kernel(const Chai
 //   warps 18 / 19        TMA producer of slot 0 / 1 (one elected lane)
 // =====================================================================================================================
 constexpr int CT_THREADS = CH_SLOTS * CH_EPI_THREADS + CH_SLOTS * 32 + CH_SLOTS * 32;  // 640
-enum { TB_IN_FULL = 0, TB_IN_FREE, TB_DA_FULL, TB_XA_FULL, TB_DB_FULL, TB_DB_FREE, TB_IN_LAND, TB_PER_SLOT };
+enum { TB_IN_FULL = 0, TB_IN_FREE, TB_DA_FULL, TB_XA_FULL, TB_DB_FULL, TB_DB_FREE, TB_PER_SLOT };
 
 struct ChainTrainParams {
     const uint8_t *w_img[2];  // P2: layers 1, 2; P3: layers 2, 3 (fp16 images, num_mg == 1)
@@ -405,10 +405,7 @@ struct ChainTrainParams {
     const float *bias_a, *mean_a, *rstd_a, *gamma_a, *beta_a;
     int dup_a;                // c_a == 64 and the first GEMM's image repeats its rows on lines 64..127 (PackJob::dup64)
     int act;
-    __half *z_out, *a_out;    // a_out NULL: only zhat is stored (one tensor per hidden layer); consumers rebuild a from it
-    // non-NULL: the fetched input tile holds zhat of the PREVIOUS layer (its a was not stored): the epilogue group turns
-    // it into a = act(gamma * zhat + beta), invalid rows 0, in shared memory before the first GEMM reads it
-    const float *fix_gamma, *fix_beta;
+    __half *z_out, *a_out;
     // second GEMM: PASS 2 -> per-channel sum / sum of squares of the bias-free accumulators, per CTA and writer group:
     // partial[(blockIdx.x * 4 + slot * 2 + half)][2][cpad]; PASS 3 -> per-centroid max (+ bias) and arg-max slot
     double *partial;
@@ -455,12 +452,10 @@ __global__ void __launch_bounds__(CT_THREADS, 1)
             mbar_init(&b[TB_XA_FULL], 1);
             mbar_init(&b[TB_DB_FULL], 1);
             mbar_init(&b[TB_DB_FREE], CH_EPI_WARPS);
-            mbar_init(&b[TB_IN_LAND], 1);
         }
         mbar_init(w_full, 1);
         fence_barrier_init();
     }
-    const bool fix_in = p.fix_gamma != nullptr;
     if (warp == CH_MMA_WARP) tmem_alloc<512>(tmem_holder);
     tc_fence_before();
     __syncthreads();
@@ -480,11 +475,10 @@ __global__ void __launch_bounds__(CT_THREADS, 1)
                 const int64_t tile = tile_of(it, s);
                 if (tile >= num_tiles) break;
                 mbar_wait(&b[TB_IN_FREE], (uint32_t)(it & 1) ^ 1u);
-                uint64_t *land = fix_in ? &b[TB_IN_LAND] : &b[TB_IN_FULL];   // a fetched zhat tile is fixed up before the MMA
-                mbar_expect_tx(land, (unsigned)in_bytes);
+                mbar_expect_tx(&b[TB_IN_FULL], (unsigned)in_bytes);
                 for (int kc = 0; kc < kc_in; ++kc)
-                    tma_load_2d(IN + kc * CH_CHUNK_BYTES, &map_in, (int)(tile * CH_ROWS), kc * KC, land);
-                mbar_arrive(land);
+                    tma_load_2d(IN + kc * CH_CHUNK_BYTES, &map_in, (int)(tile * CH_ROWS), kc * KC, &b[TB_IN_FULL]);
+                mbar_arrive(&b[TB_IN_FULL]);
             }
         }
     } else if (warp >= CH_MMA_WARP) {
@@ -605,35 +599,6 @@ __global__ void __launch_bounds__(CT_THREADS, 1)
                 nx0 = __ldg(t);
                 nx1 = __ldg(t + 1);
             }
-            if (fix_in) {
-                // ---- the fetched tile is zhat of the previous layer: a = act(gamma * zhat + beta), invalid rows 0, in place
-                unsigned nvp = 0u;   // valid rows of the tile's eight 8-row groups, 4 bits each
-#pragma unroll
-                for (int g = 0; g < 8; ++g) nvp |= (unsigned)gi_nv(dsc[g]) << (4 * g);
-                uint8_t *IN = slots + s * slot_bytes;
-                mbar_wait(&b[TB_IN_LAND], ph);
-                const int t = w8 * 32 + lane;
-                for (int c = t; c < kc_in * 512; c += CH_EPI_THREADS) {
-                    const int line = (c >> 3) & 63, kc = c >> 9;
-                    const int g = (c & 7) ^ (line & 7);               // row group held by this physical 16-byte chunk
-                    const int nv = (int)((nvp >> (4 * g)) & 15u);
-                    const int chn = kc * KC + line;
-                    const float fg = __ldg(p.fix_gamma + chn), fb = __ldg(p.fix_beta + chn);
-                    uint4 *q = reinterpret_cast<uint4 *>(IN) + c;
-                    float f[8];
-                    unpack8h(*q, f);
-#pragma unroll
-                    for (int e = 0; e < 8; ++e) {
-                        float y = fmaf(f[e], fg, fb);
-                        if (relu) y = fmaxf(y, 0.f);
-                        f[e] = e < nv ? y : 0.f;
-                    }
-                    *q = pack8h(f);
-                }
-                fence_proxy_async_smem();
-                asm volatile("bar.sync %0, %1;" ::"r"(1 + s), "n"(CH_EPI_THREADS) : "memory");
-                if (w8 == 0 && lane == 0) mbar_arrive(&b[TB_IN_FULL]);
-            }
             // ---- first GEMM: normalise; zhat and a leave through shared-memory tiles and TMA stores (16-byte global stores
             // 2*ld bytes apart per lane made this epilogue 3x slower, as they had in round 1); a is also the operand of
             // the second GEMM, read in place
@@ -694,7 +659,7 @@ __global__ void __launch_bounds__(CT_THREADS, 1)
             if (w8 == 0 && lane == 0) {
                 for (int kc = 0; kc < kc_mid; ++kc) {   // channels past c_a are clipped by the tensor maps
                     tma_store_2d(&map_z, X + x_bytes + kc * CH_CHUNK_BYTES, (int)row0, kc * KC);
-                    if (p.a_out) tma_store_2d(&map_a, X + kc * CH_CHUNK_BYTES, (int)row0, kc * KC);
+                    tma_store_2d(&map_a, X + kc * CH_CHUNK_BYTES, (int)row0, kc * KC);
                 }
                 bulk_commit_group();
                 mbar_arrive(&b[TB_XA_FULL]);
@@ -766,34 +731,19 @@ __global__ void __launch_bounds__(CT_THREADS, 1)
     if (warp == CH_MMA_WARP) tmem_dealloc<512>(tmem_base);
 }
 
-// shapes the chained training passes cover (the reference's levels 1 and 2 with neuron_multiplier 1)
-static bool chain_train_ok(const b2pn_sa_args &a, int k_img, int c1, int c2, int c3)
-{
-    if (a.seg_mode != B2PN_SEG_SLOTS || !a.training) return false;
-    if (c1 % 64 || c2 % 64 || c1 > 128 || c2 > 128 || c3 > 256 || k_img + 1 > 3 * KC) return false;
-    return true;
-}
-
 static int chain_train_smem_bytes(const ChainTrainParams &p)
 {
     return p.w_bytes[0] + p.w_bytes[1] + CH_SLOTS * (p.kc_in + 2 * p.kc_mid) * CH_CHUNK_BYTES + 256 + 1024;
 }
 
-// shapes the chained kernel covers: hidden widths of whole 64-channel chunks up to 128, output up to 256 channels, a
-// layer-1 operand of at most three 64-column chunks (the reference's levels 1 and 2 with neuron_multiplier 1)
-static bool chain_shapes_ok(const b2pn_sa_args &a, int k_img, int c1, int c2, int c3)
+// SLOTS levels whose shapes the chained kernels cover (the reference's levels 1 and 2 with neuron_multiplier 1): hidden
+// widths of whole 64-channel chunks up to 128, output up to 256 channels, and at most three 64-column chunks of the
+// layer-1 operand, `k_lines` of which the kernel reads.  The callers add the mode: evaluation with h1 == NULL
+// (tc_chain_eval_kernel), or training with g1 materialised (tc_chain_train_kernel)
+static bool chain_shapes_ok(const b2pn_sa_args &a, int k_lines, int c1, int c2, int c3)
 {
-    if (a.seg_mode != B2PN_SEG_SLOTS || a.training) return false;
-    if (c1 % 64 || c2 % 64 || c1 > 128 || c2 > 128 || c3 > 256 || k_img > 3 * KC) return false;
-    return true;
-}
-// the caller opts in by passing h1 == NULL ("I do not want the hidden activations": no backward pass will follow)
-static bool chain_eligible(const b2pn_sa_args &a, int k_img, int c1, int c2, int c3)
-{
-    if (a.h1 != nullptr) return false;
-    if (a.seg_mode != B2PN_SEG_SLOTS || a.training) return false;
-    if (c1 % 64 || c2 % 64 || c1 > 128 || c2 > 128 || c3 > 256 || k_img > 3 * KC) return false;
-    return true;
+    return a.seg_mode == B2PN_SEG_SLOTS && c1 % 64 == 0 && c2 % 64 == 0 && c1 <= 128 && c2 <= 128 && c3 <= 256 &&
+           k_lines <= 3 * KC;
 }
 
 static int chain_smem_bytes(const ChainParams &p)

@@ -407,7 +407,6 @@ struct TmaSource {
     static constexpr bool SCATTER = false;
     RowMapTC rm;
     __device__ __forceinline__ void resolve(int64_t r) { rm.resolve(r); }
-    __device__ __forceinline__ uint4 chunk_i(int, int64_t, unsigned) const { return make_uint4(0u, 0u, 0u, 0u); }
 };
 
 // The routed gradient of the max aggregation (SLOTS levels), generated on the fly instead of being stored:
@@ -425,9 +424,8 @@ struct RouteSource {
     static constexpr bool SCATTER = true;
     // The tile is zeros except for one element per (centroid that starts in it, channel): a centroid never crosses a
     // 64-row boundary, so its arg-max row is g*8 + arg inside the 64-row block its first row group g lies in.
-    // Cooperative form (what the kernels use): a loader group zeroes the tile with 16-byte stores, meets at a named
-    // barrier, then every thread drops QUADS -- 4 consecutive channels of one centroid, one 16-byte load of arg and one of
-    // dout -- at their arg-max rows.  An item costs a thread ~100 instructions instead of the ~650 of a per-line fill
+    // A loader group zeroes the tile with 16-byte stores, meets at a named barrier, then every thread drops QUADS -- 4
+    // consecutive channels of one centroid, one 16-byte load of arg and one of dout -- at their arg-max rows.  An item costs a thread ~100 instructions instead of the ~650 of a per-line fill
     // (ncu, round 2: with one loader warp per scheduler the routed kernels were bound by the loaders' dependent issue
     // latency, ~1.5 us per item, while the epilogue warps sat at their barrier 80 % of the time).
     // Needs C % 4 == 0 and 16-byte aligned arg / dout rows (`vec`, checked on the host); else four scalar loads.
@@ -476,25 +474,6 @@ struct RouteSource {
     }
     template <int NTHR = NUM_LOAD>
     static __device__ __forceinline__ void group_barrier(int id) { asm volatile("bar.sync %0, %1;" ::"r"(id), "n"(NTHR) : "memory"); }
-    // 8 rows of channel ch as one 16-byte chunk; no branch around the loads: a thread's eight (arg, dout) pairs are in
-    // flight together
-    __device__ __forceinline__ uint4 chunk_i(int ch, int64_t, unsigned inf) const
-    {
-        const bool live = ch < C && gi_nv(inf) > 0;
-        const int64_t idx = live ? (int64_t)gi_seg(inf) * C + ch : 0;
-        const int a = __ldg(arg + idx) - gi_slot0(inf);
-        const float d = __ldg(dout + idx);
-        const bool hit = live && a >= 0 && a < 8;
-        const unsigned short gb = __bfloat16_as_ushort(__float2bfloat16(d));
-        const unsigned w = (a & 1) ? ((unsigned)gb << 16) : (unsigned)gb;
-        const int q = hit ? (a >> 1) : -1;
-        uint4 v;
-        v.x = q == 0 ? w : 0u;
-        v.y = q == 1 ? w : 0u;
-        v.z = q == 2 ? w : 0u;
-        v.w = q == 3 ? w : 0u;
-        return v;
-    }
 };
 
 // MN-major B tile of the rows GEMM from a feature-major source: [2 row blocks of 64][64 channel lines];
@@ -1391,26 +1370,6 @@ struct TmaFill {
     static constexpr bool USES_TMA = true;
     int c;         // channels of the tensor; with the ones box: a multiple of 64 with (c % 256) + 16 <= 256
     int ones_box;  // 1: append the row-valid box at line c; 0: the tensor carries its own ones line (layer-1 operand)
-    // non-NULL: the tensor holds the NORMALISED values zhat and the operand wanted is the activation a = act(gamma*zhat+beta),
-    // rebuilt per channel line while the tile is converted to bf16 (only zhat is stored per hidden layer)
-    const float *fix_gamma;
-    const float *fix_beta;
-    int fix_act;
-    // 16-byte chunk c16 of the landed tile of N group ng, converted (and fixed up) in place
-    __device__ __forceinline__ uint4 convert(const uint4 &raw, int c16, int ng) const
-    {
-        const int ch = ng * 256 + (c16 >> 3);
-        if (fix_gamma == nullptr || ch >= c) return f16_to_bf16_chunk(raw);   // plain tensor / the ones box
-        const float ga = __ldg(fix_gamma + ch), be = __ldg(fix_beta + ch);
-        float f[8];
-        unpack8h(raw, f);
-#pragma unroll
-        for (int e = 0; e < 8; ++e) {
-            f[e] = fmaf(f[e], ga, be);
-            if (fix_act == B2PN_ACT_RELU) f[e] = fmaxf(f[e], 0.f);
-        }
-        return pack8(f);
-    }
     // the copies come in whole 64-line boxes: the tile must hold them even when fewer lines are used
     static __host__ __device__ int bytes(int nb_lines) { return ((nb_lines + 63) / 64) * 64 * LINE_BYTES; }
     __device__ __forceinline__ void resolve(int64_t) {}
@@ -1481,6 +1440,7 @@ __global__ void __launch_bounds__(NT, 1) tc_dw_kernel(const DwParams p, YS ys, X
                                                        const __grid_constant__ TmaMap tmap_x, const __grid_constant__ TmaMap tmap_v)
 {
     using P = DwPlan<MTA>;
+    static_assert(YS::USES_TMA || YS::SCATTER, "the Y tile comes by TMA or is built by the routed-gradient fill groups");
     // the operand ring is sized at launch: stage = A tile + the X lines actually used, as many stages as fit (<= 8) --
     // with TMA-fed operands the kernel is a pure stream and lives off the bytes it keeps in flight
     const int nst = p.stages, sbytes = p.stage_bytes;
@@ -1579,27 +1539,7 @@ __global__ void __launch_bounds__(NT, 1) tc_dw_kernel(const DwParams p, YS ys, X
                 if (lt == 0)
                     for (; iss < nchunks && iss < i + (int64_t)ahead * NG; iss += NG) issue(iss);
             }
-            if constexpr (!YS::USES_TMA) {
-                if constexpr (YS::SCATTER) {
-                    // the routed Y tile is built by the fill groups (warps 0-7, below)
-                } else {
-                    // the operand loads go out before the wait for the slot: their latency overlaps it
-                    uint4 v[MTA][8];
-#pragma unroll
-                    for (int m = 0; m < MTA; ++m) {
-                        const int ch = mg * (MTA * 128) + m * 128 + lt;
-#pragma unroll
-                        for (int g = 0; g < 8; ++g) v[m][g] = ys.chunk_i(ch, r0 + g * 8, inf[g]);
-                    }
-                    mbar_wait(&empty[s], ph ^ 1u);
-#pragma unroll
-                    for (int m = 0; m < MTA; ++m) {
-                        const int line = m * 128 + lt;
-#pragma unroll
-                        for (int g = 0; g < 8; ++g) *reinterpret_cast<uint4 *>(A + line_chunk_off(line, g)) = v[m][g];
-                    }
-                }
-            }
+            // (a routed Y tile is built by the fill groups, warps 0-7, below)
             if constexpr (XF::USES_TMA) {
                 // the stored activations are fp16, the gradients on the Y side bf16: the group converts the landed X tile
                 // to bf16 in place (16-byte chunks, element-wise: the swizzle is untouched).  Every thread first makes sure
@@ -1610,10 +1550,10 @@ __global__ void __launch_bounds__(NT, 1) tc_dw_kernel(const DwParams p, YS ys, X
                 const int nchunk16 = xf.landed_lines(ng) * 8;
                 for (int c = lt; c < nchunk16; c += NUM_LOAD) {
                     uint4 *q = reinterpret_cast<uint4 *>(B) + c;
-                    *q = xf.convert(*q, c, ng);
+                    *q = f16_to_bf16_chunk(*q);
                 }
             } else {
-                if constexpr (YS::USES_TMA || YS::SCATTER) mbar_wait(&empty[s], ph ^ 1u);  // (the in-thread Y paths have waited above)
+                mbar_wait(&empty[s], ph ^ 1u);
                 xf.fill(B, lt, r0, ng, nb_lines, inf);
             }
             fence_proxy_async_smem();
@@ -1885,7 +1825,8 @@ static void launch_pack(const float *w, int M, int Kimg, int64_t sm, int64_t sk,
 namespace b2pn {
 namespace tc {
 
-static int sm_count()
+// SM count of the current device
+static int device_sms()
 {
     static int sms_of[64] = {};  // per device; a racing first call writes the same value twice
     int dev = 0;
@@ -1896,26 +1837,33 @@ static int sm_count()
         if (sms <= 0) sms = 148;
         if (dev >= 0 && dev < 64) sms_of[dev] = sms;
     }
-    // b2pn_sa_args::sm_limit: leave SMs free for kernels of a concurrent stream (the persistent kernels below take one
-    // CTA per SM and stride over tiles by gridDim.x, so a CTA that cannot become resident would double their time)
-    const int lim = t_sm_limit;
-    return (lim > 0 && lim < sms) ? lim : sms;
+    return sms;
+}
+
+// CTAs the persistent kernels of one call may take: one per SM, or b2pn_sa_args::sm_limit, which leaves SMs free for
+// kernels of a concurrent stream (these kernels take one CTA per SM and stride over tiles by gridDim.x, so a CTA that
+// cannot become resident would double their time)
+static int cta_budget(const b2pn_sa_args &a)
+{
+    const int sms = device_sms();
+    return (a.sm_limit > 0 && a.sm_limit < sms) ? a.sm_limit : sms;
 }
 
 // grid.x of a rows-GEMM launch (the per-CTA statistics partials are indexed by blockIdx.x)
-static int grid_x_for(const Packed &pk, int64_t tiles)
+static int grid_x_for(const Packed &pk, int64_t tiles, int ctas)
 {
-    int gx = sm_count() / pk.num_mg;
+    int gx = ctas / pk.num_mg;
     if (gx < 1) gx = 1;
     if ((int64_t)gx > tiles) gx = (int)tiles;
     return gx;
 }
 
 // rows of a launch: an upper bound known on the host (sizes the grid) and, for the compacted SLOTS layout, the
-// device scalar holding the real count
+// device scalar holding the real count; and the CTAs the launch may take (cta_budget)
 struct RowsArg {
     int64_t cap;
     const int64_t *dev;
+    int ctas;
     int64_t tiles() const { return (cap + R - 1) / R; }
 };
 
@@ -1931,7 +1879,7 @@ static int launch_gemm(const Packed &pk, const RowsArg &ra, const BL &bl, const 
     cudaError_t e = ensure_dynamic_smem(kern, P::TOTAL, slot);
     if (e != cudaSuccess) return (int)e;
     GemmParams gp = {pk.img, pk.fmt, pk.fmt, pk.num_kc, ra.cap, ra.dev};
-    dim3 grid((unsigned)grid_x_for(pk, ra.tiles()), (unsigned)pk.num_mg);
+    dim3 grid((unsigned)grid_x_for(pk, ra.tiles(), ra.ctas), (unsigned)pk.num_mg);
     kern<<<grid, gemm_threads<BL>(), P::TOTAL, st>>>(gp, bl, ep, map, e0, e1);
     note_launch();
     e = cudaPeekAtLastError();
@@ -2041,14 +1989,13 @@ __global__ void bn_bwd_finalize_tc_kernel(const double *partial, int gx, int C, 
     }
 }
 
-// Routed gradient of the max aggregation as a dense feature-major bf16 tensor (SLOTS levels):
-//   dh3[ch][row] = dout[m][ch] if row is the arg-max slot of (centroid m, ch), else 0.
-// Written once so that both consumers (dX of the last layer and dW3) take it through the TMA unit instead of
-// re-deriving it per (channel, row group) in their loader warps.  Thread = (channel, 8-row group), groups fastest:
-// 16-byte stores coalesce along the rows, the (arg, dout) reads stay L2-resident.
-template <bool CLOUDS>
-__global__ void route_grad_tc_kernel(RowMapTC rm, const int64_t *rows_dev, const float *dout, const int32_t *arg, int C, int64_t ld,
-                                     __nv_bfloat16 *dh)
+// Routed gradient of the global max pool as a dense feature-major bf16 tensor (CLOUDS levels):
+//   dh3[ch][row] = dout[b][ch] if row is the arg-max source row of (cloud b = batch[row], ch), else 0.
+// Written once so that both consumers (dX of the last layer and dW3) take it through the TMA unit.  (SLOTS levels build
+// their routed tiles in the loaders instead: RouteSource.)  Thread = (channel, 8-row group), groups fastest: 16-byte stores
+// coalesce along the rows, the (arg, dout) reads stay L2-resident.
+__global__ void route_grad_clouds_tc_kernel(RowMapTC rm, const int64_t *rows_dev, const float *dout, const int32_t *arg, int C,
+                                            int64_t ld, __nv_bfloat16 *dh)
 {
     if (rows_dev) rm.rows = *rows_dev;
     const int64_t groups = (rm.rows + 127) / 128 * 16;  // whole tiles
@@ -2058,35 +2005,21 @@ __global__ void route_grad_tc_kernel(RowMapTC rm, const int64_t *rows_dev, const
         const int64_t g = i - (int64_t)ch * groups;
         const unsigned inf = rm.info(g * 8);
         uint4 v = make_uint4(0u, 0u, 0u, 0u);
-        if (CLOUDS) {  // arg names a source row of the cloud batch[row]
-            float f[8];
-            bool any = false;
+        float f[8];
+        bool any = false;
 #pragma unroll
-            for (int e = 0; e < 8; ++e) {
-                const int64_t row = g * 8 + e;
-                f[e] = 0.f;
-                if (e < gi_nv(inf)) {
-                    const int64_t sg = __ldg(rm.batch + row);
-                    if ((int64_t)__ldg(arg + sg * C + ch) == row) {
-                        f[e] = __ldg(dout + sg * C + ch);
-                        any = true;
-                    }
+        for (int e = 0; e < 8; ++e) {
+            const int64_t row = g * 8 + e;
+            f[e] = 0.f;
+            if (e < gi_nv(inf)) {
+                const int64_t sg = __ldg(rm.batch + row);
+                if ((int64_t)__ldg(arg + sg * C + ch) == row) {
+                    f[e] = __ldg(dout + sg * C + ch);
+                    any = true;
                 }
             }
-            if (any) v = pack8(f);
-        } else if (gi_nv(inf) > 0) {
-            const int64_t m = gi_seg(inf);
-            const int a = __ldg(arg + m * C + ch) - gi_slot0(inf);
-            if (a >= 0 && a < 8) {
-                const unsigned short gb = __bfloat16_as_ushort(__float2bfloat16(__ldg(dout + m * C + ch)));
-                const unsigned w = (a & 1) ? ((unsigned)gb << 16) : (unsigned)gb;
-                const int q = a >> 1;
-                v.x = q == 0 ? w : 0u;
-                v.y = q == 1 ? w : 0u;
-                v.z = q == 2 ? w : 0u;
-                v.w = q == 3 ? w : 0u;
-            }
         }
+        if (any) v = pack8(f);
         *reinterpret_cast<uint4 *>(dh + (int64_t)ch * ld + g * 8) = v;
     }
 }
@@ -2278,7 +2211,7 @@ int tc_gemm_selftest(const float *w, int m_out, int k, const void *b, int mode, 
     if (workspace_bytes < pk.bytes + 1024) return B2PN_EINVAL;
     pk.img = (uint8_t *)align_up((int64_t)(uintptr_t)workspace, 1024);
     launch_pack(w, m_out, k, k, 1, nullptr, pk, st);
-    const RowsArg ra = {rows, nullptr};
+    const RowsArg ra = {rows, nullptr, device_sms()};
     RowMapTC rm = {B2PN_SEG_CLOUDS, nullptr, nullptr, nullptr, nullptr, rows, 0};
     StoreF32Ep ep = {out, m_out, ld_out};
     if (mode == 0) {
@@ -2320,6 +2253,12 @@ struct ShapesTC {
     int64_t rows, tiles, ld;
     int c0, c1, c2, c3, cmax, cpad, k1;
     InCols cols;
+    // launch options of this call
+    int ctas;            // cta_budget(): grid bound of the persistent kernels
+    // b2pn_sa_args::deterministic.  false: the row splits of a dW GEMM add their partials into one zeroed buffer with
+    // red.global.add.v4.f32 (no partial tensor, the reduction kernel only maps columns); true: per-split partials summed
+    // in a fixed order, and the grad_x scatter of SLOTS levels accumulated in fixed point (bit-reproducible)
+    bool deterministic;
 };
 static ShapesTC shapes_tc(const b2pn_sa_args &a)
 {
@@ -2338,10 +2277,21 @@ static ShapesTC shapes_tc(const b2pn_sa_args &a)
     int mx = s.cmax > s.c3 ? s.cmax : s.c3;
     mx = mx > s.k1 + 1 ? mx : s.k1 + 1;
     s.cpad = (int)align_up(mx, 128);
+    s.ctas = cta_budget(a);
+    s.deterministic = a.deterministic != 0;
     return s;
 }
 
 constexpr int MAX_GX = 160;  // >= SM count: CTAs writing per-CTA partial buffers (4 slots each)
+
+// 1 when b2pn_sa_forward runs these arguments through the single-launch evaluation kernel if h1 == NULL (no hidden
+// activations stored)
+int sa_eval_fused_bf16(const b2pn_sa_args &a)
+{
+    if (a.mlp.c[0] != a.c_in + 3) return 0;
+    const ShapesTC s = shapes_tc(a);
+    return !a.training && chain_shapes_ok(a, s.k1, s.c1, s.c2, s.c3) ? 1 : 0;
+}
 
 static int check_args_tc(const b2pn_sa_args &a)
 {
@@ -2368,30 +2318,8 @@ static int check_args_tc(const b2pn_sa_args &a)
         if (!a.mlp.gamma[l] || !a.mlp.beta[l] || !a.mlp.running_mean[l] || !a.mlp.running_var[l]) return B2PN_EINVAL;
     if (!a.out) return B2PN_EINVAL;
     // the arg-max slots and the hidden-activation buffers are only touched by the multi-pass (training / wide-level) kernels
-    const ShapesTC sh = shapes_tc(a);
-    if (!chain_eligible(a, sh.k1, sh.c1, sh.c2, sh.c3)) {
-        if (!a.arg || !a.h1 || !a.h2 || !a.bn) return B2PN_EINVAL;
-        // the activation copies a1 / a2 are optional where the chained training kernels run (they rebuild a from zhat)
-        const bool zonly_ok = chain_train_ok(a, sh.k1, sh.c1, sh.c2, sh.c3) && a.g1 != nullptr && a.row_valid != nullptr;
-        if ((!a.a1 || !a.a2) && !(zonly_ok && !a.a1 && !a.a2)) return B2PN_EINVAL;
-    }
+    if (!(a.h1 == nullptr && sa_eval_fused_bf16(a)) && (!a.arg || !a.h1 || !a.h2 || !a.bn || !a.a1 || !a.a2)) return B2PN_EINVAL;
     return B2PN_OK;
-}
-
-// 1 when the chained TRAINING kernels cover these shapes: only zhat is stored per hidden layer, a1 / a2 may be NULL
-int sa_train_chained_bf16(const b2pn_sa_args &a)
-{
-    if (a.mlp.c[0] != a.c_in + 3) return 0;
-    const ShapesTC s = shapes_tc(a);
-    return (chain_train_ok(a, s.k1, s.c1, s.c2, s.c3) && s.k1 + 1 + 15 <= 256) ? 1 : 0;
-}
-
-// 1 when b2pn_sa_forward runs these arguments through the single-launch evaluation kernel (no hidden activations stored)
-int sa_eval_fused_bf16(const b2pn_sa_args &a)
-{
-    if (a.mlp.c[0] != a.c_in + 3) return 0;
-    const ShapesTC s = shapes_tc(a);
-    return chain_shapes_ok(a, s.k1, s.c1, s.c2, s.c3) ? 1 : 0;
 }
 
 static RowMapTC rowmap_tc(const b2pn_sa_args &a, const ShapesTC &s)
@@ -2408,7 +2336,7 @@ static RowMapTC rowmap_tc(const b2pn_sa_args &a, const ShapesTC &s)
 }
 static RowsArg rowsarg_tc(const b2pn_sa_args &a, const ShapesTC &s)
 {
-    return RowsArg{s.rows, a.seg_mode == B2PN_SEG_SLOTS ? a.num_rows : nullptr};
+    return RowsArg{s.rows, a.seg_mode == B2PN_SEG_SLOTS ? a.num_rows : nullptr, s.ctas};
 }
 
 struct FwdWsTC {
@@ -2428,18 +2356,13 @@ static FwdWsTC carve_fwd_tc(const b2pn_sa_args &a, const ShapesTC &s, WsTC &ws)
     return f;
 }
 
-// atomic mode (default): the row splits of a dW GEMM add their partials into one zeroed buffer with
-// red.global.add.v4.f32 (no partial tensor, the reduction kernel only maps columns); b2pn_sa_args::deterministic: per-split
-// partials summed in a fixed order (bit-reproducible)
-static inline bool dw_atomic() { return t_deterministic == 0; }
-
 struct DwPlanHost {
     int MTA, num_mg, num_ng, splits, nbl_total, k_stride;
     int64_t floats;
 };
 // one launch covers all (row split, M group, N group) blocks; the row range is split so that the launch fills
 // the GPU about once -- the partials the reduction has to read shrink with the size of dW
-static DwPlanHost plan_dw(int n_out, int k_total, int64_t ld)
+static DwPlanHost plan_dw(int n_out, int k_total, const ShapesTC &s)
 {
     DwPlanHost d;
     const int mpad = (int)align_up(n_out, 128);
@@ -2447,8 +2370,8 @@ static DwPlanHost plan_dw(int n_out, int k_total, int64_t ld)
     d.num_mg = (mpad + d.MTA * 128 - 1) / (d.MTA * 128);
     d.nbl_total = (int)align_up(k_total, 16);
     d.num_ng = (d.nbl_total + 255) / 256;
-    const int64_t chunks = ld / 64;
-    int sp = sm_count() / (d.num_mg * d.num_ng);
+    const int64_t chunks = s.ld / 64;
+    int sp = s.ctas / (d.num_mg * d.num_ng);
     if (sp < 1) sp = 1;
     if (sp > DWR_MAX_SPLITS) sp = DWR_MAX_SPLITS;
     if ((int64_t)sp > chunks) sp = (int)(chunks > 0 ? chunks : 1);
@@ -2480,10 +2403,10 @@ static BwdWsTC carve_bwd_tc(const b2pn_sa_args &a, const ShapesTC &s, WsTC &ws)
     // the dense routed gradient exists only at the global level (SLOTS levels generate it on the fly)
     b.dh3 = a.seg_mode == B2PN_SEG_CLOUDS ? ws.take<__nv_bfloat16>((int64_t)s.c3 * s.ld) : nullptr;
     b.sbar = ws.take<float>(2 * s.cmax);
-    b.dwp[2] = ws.take<float>(plan_dw(s.c3, s.c2 + 1, s.ld).floats);
-    b.dwp[1] = ws.take<float>(plan_dw(s.c2, s.c1 + 1, s.ld).floats);
-    b.dwp[0] = ws.take<float>(plan_dw(s.c1, s.k1 + 1, s.ld).floats);
-    b.dxi = (t_deterministic && a.seg_mode == B2PN_SEG_SLOTS && a.c_in > 0) ? ws.take<long long>(a.n_src * (int64_t)a.c_in) : nullptr;
+    b.dwp[2] = ws.take<float>(plan_dw(s.c3, s.c2 + 1, s).floats);
+    b.dwp[1] = ws.take<float>(plan_dw(s.c2, s.c1 + 1, s).floats);
+    b.dwp[0] = ws.take<float>(plan_dw(s.c1, s.k1 + 1, s).floats);
+    b.dxi = (s.deterministic && a.seg_mode == B2PN_SEG_SLOTS && a.c_in > 0) ? ws.take<long long>(a.n_src * (int64_t)a.c_in) : nullptr;
     return b;
 }
 
@@ -2531,6 +2454,40 @@ int sa_gather_rows_bf16(const b2pn_sa_args &a, cudaStream_t st)
     return B2PN_OK;
 }
 
+// BatchNorm layer l (0 or 1) of the forward: batch statistics from `nparts` partial slices (training) or the running
+// statistics -> its rows [mean, rstd, scale, shift] of the bn buffer
+static void launch_bn_fwd_finalize(const b2pn_sa_args &a, const ShapesTC &s, int l, const double *partial, int nparts,
+                                   const CountArg &count, cudaStream_t st)
+{
+    const int C = l == 0 ? s.c1 : s.c2;
+    bn_fwd_finalize_tc_kernel<<<(C + 3) / 4, 128, 0, st>>>(partial, nparts, C, s.cpad, count, a.training, a.mlp.b[l], a.mlp.gamma[l],
+                                                           a.mlp.beta[l], a.mlp.running_mean[l], a.mlp.running_var[l],
+                                                           a.mlp.num_batches_tracked[l], a.mlp.eps, a.mlp.momentum,
+                                                           a.bn + l * 4 * s.cmax, s.cmax);
+    note_launch();
+}
+
+// grid of a chained kernel (sa_chain.cuh) over `tiles64` tiles of 64 rows: CH_SLOTS tiles per CTA and round, at most the
+// call's CTA budget
+static int chain_grid(const ShapesTC &s, int64_t tiles64)
+{
+    const int64_t need = (tiles64 + CH_SLOTS - 1) / CH_SLOTS;
+    return need < s.ctas ? (int)need : s.ctas;
+}
+
+// one launch of a chained kernel; its dynamic shared memory is raised once per device (ensure_dynamic_smem)
+template <auto KERN, class... Args>
+static int launch_chain(int gx, int threads, int smem, cudaStream_t st, const Args &...args)
+{
+    static SmemAttrSlot slot = {};
+    cudaError_t e = ensure_dynamic_smem(KERN, smem, slot);
+    if (e != cudaSuccess) return (int)e;
+    KERN<<<gx, threads, smem, st>>>(args...);
+    note_launch();
+    e = cudaPeekAtLastError();
+    return e == cudaSuccess ? 0 : (int)e;
+}
+
 int sa_forward_bf16(const b2pn_sa_args &a, cudaStream_t st)
 {
     int rc = check_args_tc(a);
@@ -2546,7 +2503,8 @@ int sa_forward_bf16(const b2pn_sa_args &a, cudaStream_t st)
     float *bn1 = a.bn, *bn2 = a.bn + 4 * s.cmax;
     const int train = a.training;
 
-    const bool train_chain = a.training && s.rows > 0 && l1_materialised(a, s) && chain_train_ok(a, s.k1, s.c1, s.c2, s.c3);
+    // (the chained training kernels read g1 with its ones line)
+    const bool train_chain = a.training && s.rows > 0 && l1_materialised(a, s) && chain_shapes_ok(a, s.k1 + 1, s.c1, s.c2, s.c3);
     {
         PackJob jobs[3] = {pack_job(a.mlp.w[0], s.c1, s.k1, s.c0, 1, &s.cols, f.pk[0]),
                            pack_job(a.mlp.w[1], s.c2, s.c1, s.c1, 1, nullptr, f.pk[1]),
@@ -2558,7 +2516,7 @@ int sa_forward_bf16(const b2pn_sa_args &a, cudaStream_t st)
         jobs[1].dup64 = train_chain && s.c2 == 64;
         launch_packs(jobs, 3, st);
     }
-    if (chain_eligible(a, s.k1, s.c1, s.c2, s.c3)) {
+    if (a.h1 == nullptr && sa_eval_fused_bf16(a)) {
         // evaluation mode: the whole level in one launch, nothing but `out` written (sa_chain.cuh)
         if (s.rows == 0) return B2PN_OK;
         ChainParams cp = {};
@@ -2591,24 +2549,14 @@ int sa_forward_bf16(const b2pn_sa_args &a, cudaStream_t st)
         cp.rgrp = a.rgrp;
         GatherLoaderTC cg = {rm, a.x, s.cols, a.pos_src, a.pos_dst, -1, FMT_F16};
         const int smem = chain_smem_bytes(cp);
-        const int64_t tiles64 = (ra.cap + CH_ROWS - 1) / CH_ROWS;
-        int gx = sm_count();
-        if ((int64_t)gx * CH_SLOTS > tiles64) gx = (int)((tiles64 + CH_SLOTS - 1) / CH_SLOTS);
+        const int gx = chain_grid(s, (ra.cap + CH_ROWS - 1) / CH_ROWS);
         const int nks_last = (s.k1 - (cp.k1c - 1) * KC) >= KC ? 4 : (s.k1 - (cp.k1c - 1) * KC + 15) / 16;
-        auto launch = [&](auto kern) -> int {
-            cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-            if (e != cudaSuccess) return (int)e;
-            kern<<<gx, CH_THREADS, smem, st>>>(cp, cg);
-            return 0;
-        };
         // the reference's two levels get fully unrolled MMA issue code; anything else the run-time-shaped instance
-        if (cp.k1c == 1 && nks_last == 1 && cp.c1c == 1 && cp.c2c == 1 && cp.mt3 == 1) rc = launch(tc_chain_eval_kernel<1, 1, 1, 1, 1>);
-        else if (cp.k1c == 3 && nks_last == 1 && cp.c1c == 2 && cp.c2c == 2 && cp.mt3 == 2) rc = launch(tc_chain_eval_kernel<3, 1, 2, 2, 2>);
-        else rc = launch(tc_chain_eval_kernel<-1, -1, -1, -1, -1>);
-        if (rc) return rc;
-        note_launch();
-        B2PN_LAUNCH_CHECK();
-        return B2PN_OK;
+        if (cp.k1c == 1 && nks_last == 1 && cp.c1c == 1 && cp.c2c == 1 && cp.mt3 == 1)
+            return launch_chain<tc_chain_eval_kernel<1, 1, 1, 1, 1>>(gx, CH_THREADS, smem, st, cp, cg);
+        if (cp.k1c == 3 && nks_last == 1 && cp.c1c == 2 && cp.c2c == 2 && cp.mt3 == 2)
+            return launch_chain<tc_chain_eval_kernel<3, 1, 2, 2, 2>>(gx, CH_THREADS, smem, st, cp, cg);
+        return launch_chain<tc_chain_eval_kernel<-1, -1, -1, -1, -1>>(gx, CH_THREADS, smem, st, cp, cg);
     }
     const CountArg count = {a.seg_mode == B2PN_SEG_SLOTS ? a.num_rows + 1 : nullptr, (double)s.rows};
 
@@ -2628,30 +2576,16 @@ int sa_forward_bf16(const b2pn_sa_args &a, cudaStream_t st)
         rc = use_g1 ? launch_by_mt(f.pk[0], ra, tl1, e1, e2, st, map_g1) : launch_by_mt(f.pk[0], ra, gl, e1, e2, st);
         if (rc) return rc;
     }
-    bn_fwd_finalize_tc_kernel<<<(s.c1 + 3) / 4, 128, 0, st>>>(f.partial, ns1 * grid_x_for(f.pk[0], s.tiles), s.c1, s.cpad, count, train,
-                                                                 a.mlp.b[0], a.mlp.gamma[0], a.mlp.beta[0], a.mlp.running_mean[0],
-                                                                 a.mlp.running_var[0], a.mlp.num_batches_tracked[0], a.mlp.eps,
-                                                                 a.mlp.momentum, bn1, s.cmax);
-    note_launch();
+    launch_bn_fwd_finalize(a, s, 0, f.partial, ns1 * grid_x_for(f.pk[0], s.tiles, s.ctas), count, st);
     if (train_chain) {
         // ---- layers 1-3 in TWO chained launches (sa_chain.cuh): P2 normalises layer 1 and takes the statistics of layer 2
         // from the tile while it is in shared memory, P3 re-runs layer 2 on the stored a1, normalises, and runs layer 3 + max
-        const int64_t tiles64 = ((ra.cap + 127) / 128) * 2;
-        int gx = sm_count();
-        if ((int64_t)gx * CH_SLOTS > tiles64) gx = (int)((tiles64 + CH_SLOTS - 1) / CH_SLOTS);
-        auto launch = [&](auto kern, const ChainTrainParams &cp, const TmaMap &map) -> int {
-            const int smem = chain_train_smem_bytes(cp);
-            cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-            if (e != cudaSuccess) return (int)e;
-            TmaMap mz, ma = kNoMap;   // output maps: boxes of 64 rows x 64 channels, the layout of the shared-memory tiles
-            int r2 = make_tma_feature_major(&mz, cp.z_out, cp.c_a, cp.ld);
-            if (r2) return r2;
-            if (cp.a_out && (r2 = make_tma_feature_major(&ma, cp.a_out, cp.c_a, cp.ld))) return r2;
-            kern<<<gx, CT_THREADS, smem, st>>>(cp, map, mz, ma);
-            note_launch();
-            e = cudaPeekAtLastError();
-            return e == cudaSuccess ? 0 : (int)e;
-        };
+        const int gx = chain_grid(s, s.tiles * 2);   // whole 128-row tiles
+        // output maps of zhat / a: boxes of 64 rows x 64 channels, the layout of the shared-memory tiles
+        TmaMap mz1, ma1, mz2, ma2;
+        if ((rc = make_tma_feature_major(&mz1, z1, s.c1, s.ld)) || (rc = make_tma_feature_major(&ma1, a.a1, s.c1, s.ld)) ||
+            (rc = make_tma_feature_major(&mz2, z2, s.c2, s.ld)) || (rc = make_tma_feature_major(&ma2, a.a2, s.c2, s.ld)))
+            return rc;
         ChainTrainParams p2 = {};
         p2.w_img[0] = f.pk[0].img; p2.w_bytes[0] = (int)f.pk[0].bytes;
         p2.w_img[1] = f.pk[1].img; p2.w_bytes[1] = (int)f.pk[1].bytes;
@@ -2659,19 +2593,20 @@ int sa_forward_bf16(const b2pn_sa_args &a, cudaStream_t st)
         p2.c_a = s.c1; p2.c_b = s.c2; p2.mt_b = 1; p2.dup_a = s.c1 == 64;
         p2.rows = ra.cap; p2.rows_dev = ra.dev; p2.ld = s.ld;
         p2.bias_a = a.mlp.b[0]; p2.mean_a = bn1; p2.rstd_a = bn1 + s.cmax; p2.gamma_a = a.mlp.gamma[0]; p2.beta_a = a.mlp.beta[0];
-        p2.act = a.mlp.act; p2.z_out = (__half *)z1; p2.a_out = (__half *)a.a1;   // a_out NULL: zhat alone is stored
+        p2.act = a.mlp.act; p2.z_out = (__half *)z1; p2.a_out = (__half *)a.a1;
         p2.partial = f.partial; p2.cpad = s.cpad; p2.rgrp = a.rgrp;
+        const int smem2 = chain_train_smem_bytes(p2);
         const int nks1 = (s.k1 - (p2.kc_in - 1) * KC) >= KC ? 4 : (s.k1 - (p2.kc_in - 1) * KC + 15) / 16;
-        if (p2.kc_in == 1 && nks1 == 1 && p2.kc_mid == 1) rc = launch(tc_chain_train_kernel<2, 1, 1, 1, 1>, p2, map_g1);
-        else if (p2.kc_in == 3 && nks1 == 1 && p2.kc_mid == 2) rc = launch(tc_chain_train_kernel<2, 3, 1, 2, 1>, p2, map_g1);
-        else rc = launch(tc_chain_train_kernel<2, -1, -1, -1, -1>, p2, map_g1);
+        if (p2.kc_in == 1 && nks1 == 1 && p2.kc_mid == 1)
+            rc = launch_chain<tc_chain_train_kernel<2, 1, 1, 1, 1>>(gx, CT_THREADS, smem2, st, p2, map_g1, mz1, ma1);
+        else if (p2.kc_in == 3 && nks1 == 1 && p2.kc_mid == 2)
+            rc = launch_chain<tc_chain_train_kernel<2, 3, 1, 2, 1>>(gx, CT_THREADS, smem2, st, p2, map_g1, mz1, ma1);
+        else
+            rc = launch_chain<tc_chain_train_kernel<2, -1, -1, -1, -1>>(gx, CT_THREADS, smem2, st, p2, map_g1, mz1, ma1);
         if (rc) return rc;
-        bn_fwd_finalize_tc_kernel<<<(s.c2 + 3) / 4, 128, 0, st>>>(f.partial, 4 * gx, s.c2, s.cpad, count, train, a.mlp.b[1], a.mlp.gamma[1],
-                                                                     a.mlp.beta[1], a.mlp.running_mean[1], a.mlp.running_var[1],
-                                                                     a.mlp.num_batches_tracked[1], a.mlp.eps, a.mlp.momentum, bn2, s.cmax);
-        note_launch();
-        TmaMap map_in3;   // P3 reads a1, or -- when only zhat1 is stored -- zhat1 and rebuilds a1 in shared memory
-        if ((rc = make_tma_feature_major(&map_in3, a.a1 ? a.a1 : (const void *)z1, s.c1, s.ld))) return rc;
+        launch_bn_fwd_finalize(a, s, 1, f.partial, 4 * gx, count, st);
+        TmaMap map_in3;   // P3 reads a1
+        if ((rc = make_tma_feature_major(&map_in3, a.a1, s.c1, s.ld))) return rc;
         ChainTrainParams p3 = {};
         p3.w_img[0] = f.pk[1].img; p3.w_bytes[0] = (int)f.pk[1].bytes;
         p3.w_img[1] = f.pk[2].img; p3.w_bytes[1] = (int)f.pk[2].bytes;
@@ -2680,17 +2615,13 @@ int sa_forward_bf16(const b2pn_sa_args &a, cudaStream_t st)
         p3.rows = ra.cap; p3.rows_dev = ra.dev; p3.ld = s.ld;
         p3.bias_a = a.mlp.b[1]; p3.mean_a = bn2; p3.rstd_a = bn2 + s.cmax; p3.gamma_a = a.mlp.gamma[1]; p3.beta_a = a.mlp.beta[1];
         p3.act = a.mlp.act; p3.z_out = (__half *)z2; p3.a_out = (__half *)a.a2;
-        if (!a.a1) {
-            p3.fix_gamma = a.mlp.gamma[0];
-            p3.fix_beta = a.mlp.beta[0];
-        }
         p3.bias_b = a.mlp.b[2]; p3.out = a.out; p3.arg = a.arg; p3.out16 = (__half *)a.out_bf16; p3.rgrp = a.rgrp;
-        if (p3.kc_in == 1 && p3.kc_mid == 1 && p3.mt_b == 1) rc = launch(tc_chain_train_kernel<3, 1, 4, 1, 1>, p3, map_in3);
-        else if (p3.kc_in == 2 && p3.kc_mid == 2 && p3.mt_b == 2) rc = launch(tc_chain_train_kernel<3, 2, 4, 2, 2>, p3, map_in3);
-        else rc = launch(tc_chain_train_kernel<3, -1, -1, -1, -1>, p3, map_in3);
-        if (rc) return rc;
-        B2PN_LAUNCH_CHECK();
-        return B2PN_OK;
+        const int smem3 = chain_train_smem_bytes(p3);
+        if (p3.kc_in == 1 && p3.kc_mid == 1 && p3.mt_b == 1)
+            return launch_chain<tc_chain_train_kernel<3, 1, 4, 1, 1>>(gx, CT_THREADS, smem3, st, p3, map_in3, mz2, ma2);
+        if (p3.kc_in == 2 && p3.kc_mid == 2 && p3.mt_b == 2)
+            return launch_chain<tc_chain_train_kernel<3, 2, 4, 2, 2>>(gx, CT_THREADS, smem3, st, p3, map_in3, mz2, ma2);
+        return launch_chain<tc_chain_train_kernel<3, -1, -1, -1, -1>>(gx, CT_THREADS, smem3, st, p3, map_in3, mz2, ma2);
     }
     if (s.rows > 0) {
         NormStoreEpTC e = {s.c1, a.mlp.b[0], bn1, bn1 + s.cmax, a.mlp.gamma[0], a.mlp.beta[0], a.mlp.act, rm};
@@ -2711,11 +2642,7 @@ int sa_forward_bf16(const b2pn_sa_args &a, cudaStream_t st)
         StatsEpTC<2> e2 = {s.c2, f.partial, s.cpad, 4};
         if ((rc = launch_by_mt(f.pk[1], ra, l2, e1, e2, st, map_a1))) return rc;
     }
-    bn_fwd_finalize_tc_kernel<<<(s.c2 + 3) / 4, 128, 0, st>>>(f.partial, 4 * grid_x_for(f.pk[1], s.tiles), s.c2, s.cpad, count, train,
-                                                                 a.mlp.b[1], a.mlp.gamma[1], a.mlp.beta[1], a.mlp.running_mean[1],
-                                                                 a.mlp.running_var[1], a.mlp.num_batches_tracked[1], a.mlp.eps,
-                                                                 a.mlp.momentum, bn2, s.cmax);
-    note_launch();
+    launch_bn_fwd_finalize(a, s, 1, f.partial, 4 * grid_x_for(f.pk[1], s.tiles, s.ctas), count, st);
     if (s.rows > 0) {
         NormStoreEpTC e = {s.c2, a.mlp.b[1], bn2, bn2 + s.cmax, a.mlp.gamma[1], a.mlp.beta[1], a.mlp.act, rm};
         TmaMap mz, ma;
@@ -2745,9 +2672,9 @@ template <class YS, class XF>
 static int launch_dw(const YS &ys, const XF &xf, int n_out, int k_total, const ShapesTC &s, const RowsArg &ra, float *dwp,
                      cudaStream_t st, const TmaMap &map_y = kNoMap, const TmaMap &map_x = kNoMap, const TmaMap &map_v = kNoMap)
 {
-    const DwPlanHost d = plan_dw(n_out, k_total, s.ld);
-    DwParams p = {ra.cap, ra.dev, n_out, d.nbl_total, d.k_stride, dwp, dw_atomic() ? 1 : 0, 0, 0};
-    if (dw_atomic()) {
+    const DwPlanHost d = plan_dw(n_out, k_total, s);
+    DwParams p = {ra.cap, ra.dev, n_out, d.nbl_total, d.k_stride, dwp, s.deterministic ? 0 : 1, 0, 0};
+    if (!s.deterministic) {
         cudaError_t em = cudaMemsetAsync(dwp, 0, (size_t)n_out * d.k_stride * sizeof(float), st);
         if (em != cudaSuccess) return (int)em;
     }
@@ -2783,11 +2710,11 @@ static int launch_dw(const YS &ys, const XF &xf, int n_out, int k_total, const S
 }
 
 // grid of the element-wise BN-backward pass: grid-stride, at most 8 blocks of 256 threads per SM
-static unsigned apply_grid(int64_t ld, int C)
+static unsigned apply_grid(const ShapesTC &s, int C)
 {
-    const int64_t n = (ld / 8) * C;
+    const int64_t n = (s.ld / 8) * C;
     int64_t blocks = (n + 255) / 256;
-    const int64_t cap = (int64_t)sm_count() * 8;
+    const int64_t cap = (int64_t)s.ctas * 8;
     if (blocks > cap) blocks = cap;
     return (unsigned)(blocks > 0 ? blocks : 1);
 }
@@ -2795,8 +2722,8 @@ static unsigned apply_grid(int64_t ld, int C)
 static DwReduceJob dw_reduce_job(const float *dwp, int n_out, int k_total, const InCols *map, int k_true, int ones_idx,
                                  const ShapesTC &s, float *gw, float *gb)
 {
-    const DwPlanHost d = plan_dw(n_out, k_total, s.ld);
-    DwReduceJob j = {dwp, dw_atomic() ? 1 : d.splits, n_out, d.k_stride, map ? 1 : 0, map ? *map : InCols{0, 0}, k_true, ones_idx, gw, gb};
+    const DwPlanHost d = plan_dw(n_out, k_total, s);
+    DwReduceJob j = {dwp, s.deterministic ? d.splits : 1, n_out, d.k_stride, map ? 1 : 0, map ? *map : InCols{0, 0}, k_true, ones_idx, gw, gb};
     return j;
 }
 static void launch_dw_reduces(const DwReduceJob *jobs, int n, cudaStream_t st)
@@ -2853,14 +2780,11 @@ int sa_backward_bf16(const b2pn_sa_args &a, const b2pn_sa_grads &g, cudaStream_t
     if (tma_x2 || tma_x1) {
         if ((rc = make_tma_row_valid(&map_v, a.row_valid, s.ld))) return rc;
     }
-    // only zhat stored (a1 == NULL, chained training path): the X sides read zhat and rebuild a in shared memory
-    const bool x_from_z = a.a1 == nullptr;
-    if (x_from_z && !(tma_x1 && tma_x2 && a.seg_mode == B2PN_SEG_SLOTS)) return B2PN_EINVAL;
-    if (tma_x2 && (rc = make_tma_feature_major(&map_a2, x_from_z ? (const void *)z2 : a.a2, s.c2, s.ld))) return rc;
-    if (tma_x1 && (rc = make_tma_feature_major(&map_a1, x_from_z ? (const void *)z1 : a.a1, s.c1, s.ld))) return rc;
+    if (tma_x2 && (rc = make_tma_feature_major(&map_a2, a.a2, s.c2, s.ld))) return rc;
+    if (tma_x1 && (rc = make_tma_feature_major(&map_a1, a.a1, s.c1, s.ld))) return rc;
     if (a.seg_mode == B2PN_SEG_CLOUDS) {
         // global level (few rows): materialise dh3 once, then both consumers read it through TMA
-        route_grad_tc_kernel<true><<<apply_grid(s.ld, s.c3), 256, 0, st>>>(rm, ra.dev, g.grad_out, a.arg, s.c3, s.ld, b.dh3);
+        route_grad_clouds_tc_kernel<<<apply_grid(s, s.c3), 256, 0, st>>>(rm, ra.dev, g.grad_out, a.arg, s.c3, s.ld, b.dh3);
         note_launch();
         TmaMap map3;
         if ((rc = make_tma_feature_major(&map3, b.dh3, s.c3, s.ld))) return rc;
@@ -2868,7 +2792,7 @@ int sa_backward_bf16(const b2pn_sa_args &a, const b2pn_sa_grads &g, cudaStream_t
         if ((rc = launch_by_mt(b.pkT[2], ra, bl, e31, e32, st, map3, mdz2, mz2))) return rc;          // da2 = W3^T dh3
         TmaSource y3 = {rm};
         if (tma_x2) {
-            TmaFill xt = {s.c2, 1, nullptr, nullptr, 0};
+            TmaFill xt = {s.c2, 1};
             rc = launch_dw(y3, xt, s.c3, s.c2 + 1, s, ra, b.dwp[2], st, map3, map_a2, map_v);   // dW3 = dh3^T a2
         } else {
             rc = launch_dw(y3, xa2, s.c3, s.c2 + 1, s, ra, b.dwp[2], st, map3);
@@ -2882,18 +2806,18 @@ int sa_backward_bf16(const b2pn_sa_args &a, const b2pn_sa_grads &g, cudaStream_t
         FeatLoaderTC<RouteSource, true> bl = {rs};
         if ((rc = launch_by_mt(b.pkT[2], ra, bl, e31, e32, st, kNoMap, mdz2, mz2))) return rc;        // da2 = W3^T dh3
         if (tma_x2) {
-            TmaFill xt = {s.c2, 1, x_from_z ? a.mlp.gamma[1] : nullptr, a.mlp.beta[1], a.mlp.act};
+            TmaFill xt = {s.c2, 1};
             rc = launch_dw(rs, xt, s.c3, s.c2 + 1, s, ra, b.dwp[2], st, kNoMap, map_a2, map_v);  // dW3 = dh3^T a2
         } else {
             rc = launch_dw(rs, xa2, s.c3, s.c2 + 1, s, ra, b.dwp[2], st);
         }
         if (rc) return rc;
     }
-    bn_bwd_finalize_tc_kernel<<<(s.c2 + 3) / 4, 128, 0, st>>>(b.partial, 4 * grid_x_for(b.pkT[2], s.tiles), s.c2, s.cpad, count,
+    bn_bwd_finalize_tc_kernel<<<(s.c2 + 3) / 4, 128, 0, st>>>(b.partial, 4 * grid_x_for(b.pkT[2], s.tiles, s.ctas), s.c2, s.cpad, count,
                                                                  a.training, g.grad_gamma[1], g.grad_beta[1], b.sbar);
     note_launch();
     {
-        bn_bwd_apply_tc_kernel<<<apply_grid(s.ld, s.c2), 256, 0, st>>>(rm, ra.dev, b.dz2, z2, s.c2, s.ld, bn2 + 2 * s.cmax, b.sbar);
+        bn_bwd_apply_tc_kernel<<<apply_grid(s, s.c2), 256, 0, st>>>(rm, ra.dev, b.dz2, z2, s.c2, s.ld, bn2 + 2 * s.cmax, b.sbar);
         note_launch();
     }
     // ---- layer 2 ---------------------------------------------------------------------------------------
@@ -2911,7 +2835,7 @@ int sa_backward_bf16(const b2pn_sa_args &a, const b2pn_sa_grads &g, cudaStream_t
         if ((rc = make_tma_feature_major(&mz1, z1, s.c1, s.ld, 32))) return rc;
         if ((rc = launch_by_mt(b.pkT[1], ra, bl, e1, e2, st, map2, mdz1, mz1))) return rc;
         if (tma_x1) {
-            TmaFill xt = {s.c1, 1, x_from_z ? a.mlp.gamma[0] : nullptr, a.mlp.beta[0], a.mlp.act};
+            TmaFill xt = {s.c1, 1};
             rc = launch_dw(y2, xt, s.c2, s.c1 + 1, s, ra, b.dwp[1], st, map2, map_a1, map_v);
         } else {
             LineFillK<FeatSource<1>> xa1 = {{rm, z1, s.c1, s.ld, a.mlp.act, s.c1, a.mlp.gamma[0], a.mlp.beta[0], FMT_BF16}};
@@ -2919,11 +2843,11 @@ int sa_backward_bf16(const b2pn_sa_args &a, const b2pn_sa_grads &g, cudaStream_t
         }
         if (rc) return rc;
     }
-    bn_bwd_finalize_tc_kernel<<<(s.c1 + 3) / 4, 128, 0, st>>>(b.partial, 4 * grid_x_for(b.pkT[1], s.tiles), s.c1, s.cpad, count,
+    bn_bwd_finalize_tc_kernel<<<(s.c1 + 3) / 4, 128, 0, st>>>(b.partial, 4 * grid_x_for(b.pkT[1], s.tiles, s.ctas), s.c1, s.cpad, count,
                                                                  a.training, g.grad_gamma[0], g.grad_beta[0], b.sbar);
     note_launch();
     {
-        bn_bwd_apply_tc_kernel<<<apply_grid(s.ld, s.c1), 256, 0, st>>>(rm, ra.dev, b.dz1, z1, s.c1, s.ld, bn1 + 2 * s.cmax, b.sbar);
+        bn_bwd_apply_tc_kernel<<<apply_grid(s, s.c1), 256, 0, st>>>(rm, ra.dev, b.dz1, z1, s.c1, s.ld, bn1 + 2 * s.cmax, b.sbar);
         note_launch();
     }
     // ---- layer 1 ---------------------------------------------------------------------------------------
@@ -2932,7 +2856,7 @@ int sa_backward_bf16(const b2pn_sa_args &a, const b2pn_sa_grads &g, cudaStream_t
         if (l1_materialised(a, s)) {
             TmaMap map_g1;
             if ((rc = make_tma_feature_major(&map_g1, a.g1, s.k1 + 1, s.ld))) return rc;
-            TmaFill xt = {s.k1 + 1, 0, nullptr, nullptr, 0};
+            TmaFill xt = {s.k1 + 1, 0};
             rc = launch_dw(y1, xt, s.c1, s.k1 + 1, s, ra, b.dwp[0], st, map1, map_g1, kNoMap);
         } else {
             LineFillGather xg = {{rm, a.x, s.cols, a.pos_src, a.pos_dst, s.k1, FMT_BF16}};  // X side of dW1: meets bf16 gradients

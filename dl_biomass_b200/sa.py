@@ -17,12 +17,6 @@ from . import _lib
 from .optim import fresh_alias, grad_dst
 
 PREC_F32, PREC_BF16 = 0, 1
-# True: the chained training kernels keep ONE tensor per hidden layer (zhat) and rebuild the activation a = act(gamma*zhat
-# + beta) where it is needed (forward P3, the X side of the dW GEMMs): half the activation memory and two tensor writes
-# fewer per level, but MEASURED SLOWER on B200 (12 x 10k points: 2.44 vs 2.31 ms/step -- the in-shared-memory fix-up costs
-# the consumers more than the stores cost the producer: P3 128 -> 159 us, dW 43-100 -> 54-112 us), so the default stores
-# the activation copies as well
-STORE_ZHAT_ONLY = False
 
 # storage format of the FORWARD-domain 16-bit tensors of the tensor-core mode (weights, normalised activations, level
 # outputs handed to the next level): fp16 -- 8x finer than bf16 on O(1) values, which the 2e-2 output tolerance needs at
@@ -285,16 +279,7 @@ class _SAFunction(torch.autograd.Function):
             ld = (rows + 127) // 128 * 128
             h1 = torch.empty(chans[1], ld, dtype=H16, device=dev)
             h2 = torch.empty(chans[2], ld, dtype=H16, device=dev)
-            zonly = False
-            if training and seg_mode == SEG_SLOTS and STORE_ZHAT_ONLY:
-                probe = SaArgs()
-                probe.precision, probe.training, probe.seg_mode, probe.K, probe.c_in = prec, 1, seg_mode, K, c_in
-                probe.x_dtype = 0 if (x is not None and x.dtype == f32 and c_in <= 16) else 1
-                for i in range(4):
-                    probe.mlp.c[i] = chans[i]
-                zonly = lib.b2pn_sa_train_chained(ctypes.byref(probe)) == 1
-            # post-activation copies (TMA operands) -- not where the chained training kernels rebuild them from zhat
-            acts = [None, None] if zonly else [torch.empty_like(h1), torch.empty_like(h2)]
+            acts = [torch.empty_like(h1), torch.empty_like(h2)]   # post-activation copies (TMA operands)
             if seg_mode == SEG_CLOUDS:   # the "ones" operand line of the dW GEMMs: 1 on every real row
                 rowmap = (None, None, None, 0, _row_valid_clouds(ld, n_src, dev))
             if seg_mode == SEG_SLOTS and k_img + 16 <= 256:   # gathered layer-1 operand incl. its ones line

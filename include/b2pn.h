@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define B2PN_ABI_VERSION 6
+#define B2PN_ABI_VERSION 7
 #define B2PN_OK 0
 #define B2PN_EINVAL (-1)   /* null pointer / negative size / bad flag            */
 #define B2PN_ENOTSUP (-2)  /* shape outside what the sm_100a kernels are built for */
@@ -195,8 +195,8 @@ typedef struct b2pn_sa_args {
     const void *row_valid;       /* fp16 [row_capacity] from b2pn_pack_rows, or NULL                    */
     /* PREC_BF16: activations of the two hidden layers AFTER BatchNorm affine + activation, fp16 feature-major
      * [c, ld] like h1/h2, invalid rows zero.  Written by forward, read by backward: stored next to the
-     * normalised values so that every later consumer is a plain tensor-map (TMA) copy.  OPTIONAL (both NULL) where
-     * b2pn_sa_train_chained() == 1: those kernels rebuild a from the normalised values.                  */
+     * normalised values so that every later consumer is a plain tensor-map (TMA) copy.  Required whenever
+     * h1 != NULL.                                                                                        */
     void *a1, *a2;
     /* PREC_BF16 + SEG_SLOTS, optional (NULL = gather in the loader warps): the gathered + concatenated layer-1
      * operand, fp16 feature-major [c_img + 1, ld] with c_img = (x fp32 ? 2 : 1) * c_in + 6 image columns
@@ -240,10 +240,6 @@ int b2pn_sa_forward(const b2pn_sa_args *args, b2pn_stream_t stream);
  * are not touched either -- arg may be NULL -- and no backward pass can follow); with h1 != NULL the multi-pass kernels run
  * and fill them.  0 otherwise. */
 int b2pn_sa_eval_fused(const b2pn_sa_args *args);
-/* 1 if, in TRAINING mode, these shapes go through the chained kernels (three GEMM passes per level, two layers per launch).
- * They store ONE tensor per hidden layer -- the normalised values h1 / h2 -- and rebuild the activations from it wherever
- * they are needed (forward P3, backward dW): the caller may pass a1 == a2 == NULL (g1 and row_valid are then required). */
-int b2pn_sa_train_chained(const b2pn_sa_args *args);
 /* PREC_BF16 + SEG_SLOTS: only the gather + concat of /root/reference/pointnet2_regressor.py:17-18's message inputs
  * ([x_j | pos_j - pos_i]) into args->g1.  Needs x, pos_src, pos_dst, the compacted rows and c_in / mlp.c[0..1]; no
  * weights, no workspace: a caller may run it ahead of the forward pass (e.g. for the next batch on another stream).

@@ -114,6 +114,16 @@ def test_host_side_sizing_helpers(built_lib):
     neg = built_lib.SaArgs()                                  # launch options are per-call fields, checked per call
     neg.precision, neg.sm_limit = 1, -3
     assert h.b2pn_sa_forward(ctypes.byref(neg), None) == -1 and h.b2pn_sa_workspace_bytes(ctypes.byref(neg), 0) == -1
+    lvl = built_lib.SaArgs()                                  # a SLOTS level with features: the backward's workspace
+    lvl.precision, lvl.seg_mode, lvl.K, lvl.n_src, lvl.n_dst, lvl.c_in = 1, 0, 64, 10000, 1000, 1
+    lvl.row_capacity = h.b2pn_pack_rows_capacity(1000, 64)
+    for i, c in enumerate((4, 64, 64, 128)):
+        lvl.mlp.c[i] = c
+    fast = h.b2pn_sa_workspace_bytes(ctypes.byref(lvl), 1)
+    lvl.deterministic = 1                                     # + the fixed-point grad_x accumulator, this call only
+    assert h.b2pn_sa_workspace_bytes(ctypes.byref(lvl), 1) >= fast + 10000 * 8 > fast > 0
+    lvl.deterministic = 0
+    assert h.b2pn_sa_workspace_bytes(ctypes.byref(lvl), 1) == fast
     nm = subprocess.run(["nm", "-D", "--defined-only", built_lib.LIB_PATH], capture_output=True, text=True).stdout
     assert "b2pn_set_" not in nm and "set_variant" not in nm   # no process-wide setters left in the ABI
     assert h.b2pn_head_forward(None, None) == -1 and h.b2pn_head_backward(None, None, None) == -1

@@ -247,19 +247,6 @@ def test_pinned_slots_options(cuda_device, case, opts):
     run_level(name, cuda_device, c_in=c["c_in"], chans=c["chans"], K=c["K"], problem=prob, **opts).finish()
 
 
-@pytest.mark.parametrize("case", ["ref_l1", "ref_l2"])
-def test_pinned_zhat_only(cuda_device, monkeypatch, case):
-    """sa.STORE_ZHAT_ONLY: the chained kernels keep zhat alone; P3 rebuilds a1 (fix_gamma), the dW X sides rebuild a."""
-    monkeypatch.setattr(sa, "STORE_ZHAT_ONLY", True)
-    c = dict(SLOTS_CASES[case])
-    prob = _slots_problem(c["c_in"], c["chans"], c["K"], c["B"], c["n"], c["r"], 21, cuda_device)
-    if c["c_in"] > 16:
-        prob = (prob[0].half().float(),) + prob[1:]
-    rep = run_level(case + "/zhat_only", cuda_device, c_in=c["c_in"], chans=c["chans"], K=c["K"], problem=prob)
-    assert rep.state["a1"] is None and rep.state["a2"] is None
-    rep.finish()
-
-
 @pytest.mark.parametrize("n_dst,tail", [(160, "rows = 20 x 64, last 128-row tile full"),
                                         (161, "rows = 21 x 64, last 128-row tile half used"),
                                         (159, "rows = 20 x 64, last group of the last tile short")])
