@@ -351,7 +351,7 @@ __global__ void __launch_bounds__(CH_THREADS, 1) tc_chain_eval_kernel(const Chai
 #pragma unroll
                             for (int e = 0; e < 8; ++e)
                                 if (e < nv) best = fmaxf(best, v[gg * 8 + e]);
-                            bk = 0;
+                            if (nv > 0) bk = 0;   // an empty neighbourhood (cnt = 0: one group, nv = 0) stays 0
                         }
                         if (gi_last(inf) && ch3 < p.c3) {
                             const int64_t m = gi_seg(inf);

@@ -174,7 +174,9 @@ typedef struct b2pn_sa_args {
     const float *pos_src;        /* [n_src, 3]                                                        */
     const float *pos_dst;        /* [n_dst, 3] (SLOTS) / NULL (CLOUDS: centre is the origin)          */
     const int32_t *nbr;          /* [n_dst, K] (SLOTS)                                                */
-    const int32_t *cnt;          /* [n_dst]    (SLOTS)                                                */
+    const int32_t *cnt;          /* [n_dst]    (SLOTS); cnt[m] = 0 is allowed: an empty neighbourhood gives
+                                    out[m] = 0 (and arg -1) on every path -- fp32, multi-pass 16-bit and the
+                                    single-launch evaluation kernel -- as PyG's max aggregation of no messages */
     const int64_t *batch;        /* [n_src] sorted cloud id per row (CLOUDS)                          */
     b2pn_mlp3 mlp;
     float *out;                  /* [n_dst, c3]                                                       */
