@@ -346,6 +346,7 @@ __global__ void __launch_bounds__(HEAD_THREADS, 1) head_backward_kernel(const b2
 static int head_check(const b2pn_head_args &a, bool forward)
 {
     if (a.B <= 0 || a.B > HEAD_MAX_B) return a.B <= 0 ? B2PN_EINVAL : B2PN_ENOTSUP;
+    if (a.training && a.B < 2) return B2PN_EINVAL;  // batch statistics of one row: BatchNorm1d refuses to train on it
     if (a.c[0] <= 0 || a.c[1] <= 0 || a.c[2] <= 0 || a.c[3] <= 0) return B2PN_EINVAL;
     if (a.c[1] > HEAD_MAX_C || a.c[2] > HEAD_MAX_C || a.c[3] > HEAD_MAX_OUT) return B2PN_ENOTSUP;
     if (!(a.p >= 0.f && a.p < 1.f)) return B2PN_EINVAL;

@@ -114,6 +114,8 @@ def head_apply(mlp, x: torch.Tensor, counter: torch.Tensor, seed: int) -> torch.
     l0, l1, l2 = mlp.lins
     n0, n1 = mlp.norms
     params = (l0.weight, l0.bias, n0.weight, n0.bias, l1.weight, l1.bias, n1.weight, n1.bias, l2.weight, l2.bias)
+    if mlp.training and x.size(0) < 2:   # as torch's BatchNorm1d: one row has no batch variance to normalise with
+        raise ValueError(f"Expected more than 1 value per channel when training, got input size {tuple(x.shape)}")
     if x.size(0) > MAX_ROWS:
         if mlp.training:
             raise ValueError(f"the fused head trains on at most {MAX_ROWS} clouds per batch")

@@ -253,6 +253,8 @@ int b2pn_sa_backward(const b2pn_sa_args *args, const b2pn_sa_grads *grads, b2pn_
  * Regression head: the MLP([c0, c1, c2, c3], act=None, dropout=p) of /root/reference/pointnet2_regressor.py:50,58
  * (torch_geometric.nn.MLP: Lin -> BatchNorm1d -> dropout -> Lin -> BatchNorm1d -> dropout -> Lin) on B <= 32 rows,
  * one forward and one backward kernel instead of ~60 ATen launches.  fp32.  c1, c2 <= 256, c3 <= 8.
+ * Training needs B >= 2 (B2PN_EINVAL otherwise): like torch's BatchNorm1d, the head does not normalise one row by
+ * its own zero variance.
  * Dropout noise is counter based: (seed, *rng_counter, layer, element); forward bumps *rng_counter when training,
  * which keeps the op replayable from a CUDA graph.
  * ---------------------------------------------------------------------------------------------- */

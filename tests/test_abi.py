@@ -64,7 +64,8 @@ def test_product_never_imports_oracle():
 def test_oracle_never_imports_product():
     """The oracle is an independent restatement: oracle/ref.py and oracle/augment_ref.py must not lean on the package they
     check (the golden-vector generator scripts may use its synthetic-cloud helper)."""
-    for f in ("ref.py", "augment_ref.py", "sa_pinned.py", "sa_eval_ref.py", "b2pn_oracle.c"):
+    for f in ("ref.py", "augment_ref.py", "sa_pinned.py", "sa_eval_ref.py", "sa_f32_pinned.py", "head_ref.py",
+              "b2pn_oracle.c"):
         txt = open(os.path.join(ROOT, "oracle", f)).read()
         assert not re.search(r"^\s*(from|import)\s+dl_biomass_b200\b", txt, flags=re.M), f
         assert "libb2pn.so" not in txt, f
@@ -135,3 +136,7 @@ def test_host_side_sizing_helpers(built_lib):
     for i, c in enumerate((1024, 128, 128, 4)):
         a.c[i] = c
     assert h.b2pn_head_forward(ctypes.byref(a), None) == -2
+    a.B, a.training = 1, 1                                    # batch statistics of one row: refused like BatchNorm1d
+    assert h.b2pn_head_forward(ctypes.byref(a), None) == -1
+    g = built_lib.HeadGrads()
+    assert h.b2pn_head_backward(ctypes.byref(a), ctypes.byref(g), None) == -1
